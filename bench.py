@@ -12,6 +12,8 @@ series.  A step = one full scan+decode+filter+dedup+aggregate pass over all of t
   cpu_baseline : the CPU oracle (C restatement of the reference path) on a bounded sample, all host threads.
 
 `--impl reference` times that CPU restatement alone (the reference itself is Rust and cannot be built here).
+`--dump-outputs DIR` writes the result of the last timed step (series_id, count, sum, min, max of every group) as float64
+DIR/<column>.npy; the inputs are seeded, so two builds run with the same arguments can be compared output for output.
 """
 import argparse
 import ctypes as C
@@ -172,6 +174,31 @@ def check_parity(tbl, exp):
     return bool(ok)
 
 
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def unpack_outputs(block):
+    """[6, n] packed aggregate (key, bucket, count, sum / min / max bits; count == 0 pads) -> the result columns a caller of
+    scan_aggregate receives for this query (no time buckets), as float64 (series ids and counts stay below 2**53)."""
+    live = block[2] > 0
+    f64 = lambda r: np.ascontiguousarray(block[r][live]).view(np.float64)
+    return {"series_id": block[0][live].astype(np.float64), "count": block[2][live].astype(np.float64),
+            "sum": f64(3), "min": f64(4), "max": f64(5)}
+
+
+def dump_outputs(out_dir, cols):
+    """One DIR/<name>.npy per column.  Above DUMP_LIMIT_BYTES in all, a fixed seeded sample of the groups is kept, in result
+    order, and `row_index` records which rows it holds."""
+    n = len(cols["count"])
+    keep = DUMP_LIMIT_BYTES // (8 * (len(cols) + 1)) - 16        # room for row_index and the .npy headers
+    if n > keep:
+        idx = np.sort(np.random.default_rng(0).choice(n, keep, replace=False))
+        cols = {"row_index": idx.astype(np.float64), **{k: v[idx] for k, v in cols.items()}}
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in cols.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.ascontiguousarray(a, dtype=np.float64))
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -184,7 +211,11 @@ def main():
     ap.add_argument("--e2e-steps", type=int, default=3)
     ap.add_argument("--no-variant", action="store_true", help="skip the secondary codec measurement")
     ap.add_argument("--no-compaction", action="store_true", help="skip the merge-compaction variant (N=1 only, own process)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the last timed step's result (all GPUs' groups, main codec) as DIR/<column>.npy in float64")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
 
     # stdout carries exactly ONE JSON line: route everything else (NCCL banners, library chatter) to stderr
     real_stdout = os.dup(1)
@@ -360,6 +391,14 @@ def main():
         ev1.record(stream)
         barrier()
         ms = ev0.elapsed_time(ev1)
+        # the last timed step's device result, packed before any later call replaces the engine's last aggregate
+        g_local = int(dev.num_groups)
+        cap = max(g_local, 1)
+        blk = torch.empty(6, cap, device="cuda", dtype=torch.int64)     # pack_agg writes all `cap` columns
+        with torch.cuda.stream(stream):
+            eng.export_packed(blk.data_ptr(), cap)
+        stream.synchronize()
+        own = blk.cpu().numpy()
         if world > 1:
             last = gathered_block(last)
         if rank == 0:
@@ -374,19 +413,14 @@ def main():
             ms = float(tt.item())
         st = eng.stats()
         # ---- parity of the TIMED configuration: the last timed step's device result against the oracle
-        g_local = int(dev.num_groups)
-        cap = max(g_local, 1)
-        blk = torch.zeros(6, cap, device="cuda", dtype=torch.int64)
-        with torch.cuda.stream(stream):
-            eng.export_packed(blk.data_ptr(), cap)
-        stream.synchronize()
-        own = blk.cpu().numpy()
         parity_resident = packed_matches(own, expected)
         parity_combined = None
+        outputs = unpack_outputs(own)
         if world > 1:
             # every rank's slot of the gathered block must carry exactly that rank's partial (checked through checksums of
             # the ranks' ORACLE results), and this rank's slot must equal its own oracle result bit for bit
             gathered = last.cpu().numpy()                       # [world, 6, cap]
+            outputs = unpack_outputs(np.concatenate(list(gathered), axis=1))   # every rank's groups, rank by rank
             mine = gathered[rank]
             ok = packed_matches(mine, expected)
             exp_blk = np.zeros((6, len(expected.count)), dtype=np.int64)
@@ -419,12 +453,14 @@ def main():
                 "ungated_kernel_ms": ungated_ms,"rows": rows, "file_bytes": file_bytes, "ms_total": ms, "ms_per_step": ms / steps, "kernel_ms": float(np.mean(kernel_ms)),
                 "call_ms": float(np.mean(call_ms)), "launches": launches, "e2e_s": e2e_dt, "d2h": d2h, "h2d": h2d, "stats": st,
                 "groups": total_groups, "groups_local": groups_local,
-                "clocks": sampler.summary() if rank == 0 else None, "ssts": ssts}
+                "clocks": sampler.summary() if rank == 0 else None, "ssts": ssts, "outputs": outputs}
 
     res = {c: measure(c, args.steps, args.warmup, args.e2e_steps) for c in codecs}
     main_r = res[args.codec]
 
     if rank == 0:
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, main_r["outputs"])
         peaks = {}
         try:
             peaks = json.load(open(os.path.join(ROOT, "MEASURED_PEAKS.json")))
