@@ -73,6 +73,10 @@ class HgWriteProps(C.Structure):
     _fields_ = [("max_row_group_size", C.c_uint32), ("compression", C.c_uint32), ("enable_sorting_columns", C.c_uint32), ("_pad", C.c_uint32)]
 
 
+# codec names of the GPU writer -> Parquet codec ids (hg_write_props.compression)
+_CODECS = {"none": 0, "uncompressed": 0, "snappy": 1, "zstd": 6}
+
+
 class HgFileMeta(C.Structure):
     _fields_ = [("size", C.c_uint64), ("num_rows", C.c_uint32), ("_pad", C.c_uint32), ("time_start", C.c_int64), ("time_end", C.c_int64),
                 ("max_sequence", C.c_uint64)]
@@ -303,7 +307,7 @@ class Engine:
         `shard_preds` = this GPU's pk0 range in a multi-GPU compaction (see `plan_pk_splitters`)."""
         arr, keep = self._descs(ssts)
         p = _make_preds(schema.arrow_schema, shard_preds)
-        props = HgWriteProps(max_row_group_size, {"none": 0, "uncompressed": 0, "snappy": 1}[compression.lower()], int(enable_sorting_columns), 0)
+        props = HgWriteProps(max_row_group_size, _CODECS[compression.lower()], int(enable_sorting_columns), 0)
         meta = HgFileMeta()
         _check(self._L.hg_compact_to_sst(self._h, C.byref(schema.desc), arr, C.c_size_t(len(ssts)), p, C.c_size_t(len(shard_preds)), C.byref(props),
                                          out_path.encode(), C.byref(meta)))
@@ -325,7 +329,7 @@ class Engine:
 
         carr = _CArray()
         st._export_to_c(C.addressof(carr))
-        props = HgWriteProps(max_row_group_size, {"none": 0, "uncompressed": 0, "snappy": 1}[compression.lower()], int(enable_sorting_columns), 0)
+        props = HgWriteProps(max_row_group_size, _CODECS[compression.lower()], int(enable_sorting_columns), 0)
         meta = HgFileMeta()
         try:
             _check(self._L.hg_write_batch(self._h, C.byref(schema.desc), C.byref(carr), C.c_uint64(sequence), C.byref(props), out_path.encode(), C.byref(meta)))

@@ -2,8 +2,8 @@
 // (compaction/executor.rs:173-203: AsyncArrowWriter over the merged stream) and of write_batch (storage.rs:189-225), with
 // the writer properties of build_write_props (storage.rs:258-298) and WriteConfig::default (config.rs:120-133):
 // row groups of max_row_group_size rows, one DataPage V1 per column chunk, PLAIN values, RLE/bit-packed definition levels
-// (every field is nullable), dictionary off, bloom filters off, chunk statistics (min / max / null_count), Snappy or
-// uncompressed pages, sorting_columns = primary keys ascending nulls first, Thrift-compact footer.
+// (every field is nullable), dictionary off, bloom filters off, chunk statistics (min / max / null_count), Snappy,
+// Zstandard or uncompressed pages, sorting_columns = primary keys ascending nulls first, Thrift-compact footer.
 //
 // Device work: page bodies (level prefix + compacted non-null values), chunk statistics, page compression and the final
 // gather into one contiguous file image.  Host work: the few KB of Thrift (page headers, footer) and the offsets.
@@ -13,6 +13,13 @@
 // copies of the agreeing high bytes (offset = value width) and 64-byte run-length copies.  Every value computes its own
 // emitted size, one prefix sum gives all positions, every value writes its own bytes: no serial parse, any Snappy decoder
 // reads the result.  (On the synthetic metric data it lands within a few percent of the reference compressor's ratio.)
+//
+// The Zstandard compressor (RFC 8878) sees the same values, with one more match source: a per-block hash table finds an
+// earlier equal value further back (in a timestamp column: the same timestamp one series earlier), and consecutive values
+// that match at the same distance become one long match.  Every sequence uses an explicit offset (never a repeat code), so
+// the 128 KB blocks of a page are independent and compress in parallel, one CTA each.  Literals are stored raw; literal
+// lengths, match lengths and offsets are entropy coded (RLE / predefined / FSE tables chosen per block by estimated size).
+// The code tables are the decoder's (zstd_core.h).  A block that would not shrink is stored as a Raw block.
 #include <cuda_runtime.h>
 
 #include <algorithm>
@@ -22,6 +29,25 @@
 
 #include "engine_internal.h"
 #include "sst_writer.h"
+
+// zstd_core.h's primitives (the decoder itself is not used here: only its code tables and predefined distributions)
+#define SNP_FN __device__ __forceinline__
+#define SNP_CONST __constant__ const
+#define snp_any(p) __any_sync(0xffffffffu, (p))
+#define snp_syncwarp() __syncwarp()
+#define snp_ldg8(p) __ldg(p)
+#define snp_ldcg8(p) (*(p))
+#define snp_set_err(err, code) atomicExch((err), (code))
+namespace horae {
+namespace zst {
+__device__ __forceinline__ uint64_t snp_ldg64u(const uint8_t* p) {
+  uint64_t v = 0;
+  for (int i = 0; i < 8; i++) v |= uint64_t(__ldg(p + i)) << (8 * i);
+  return v;
+}
+}  // namespace zst
+}  // namespace horae
+#include "zstd_core.h"
 
 namespace horae {
 namespace writer {
@@ -325,6 +351,384 @@ __global__ void __launch_bounds__(kThreads) snappy_encode_kernel(const uint8_t* 
   }
 }
 
+// ------------------------------------------------------------------------------------------------ Zstandard compression
+constexpr uint32_t kZBlk = zst::kBlockMax;      // bytes of page content per block
+constexpr int kZHashLog = 13;                   // per-block table of earlier values: 8192 slots, the most recent index wins
+constexpr uint32_t kZFront = 16;                // room in front of block 0 for the frame header
+constexpr uint32_t kZPad = 512;                 // slot bytes beyond the block content: block / literal / sequence headers, tables
+constexpr uint32_t kZArrays = 10;               // u32 scratch arrays per CTA, one entry per value of the block (+1)
+
+// frame header: magic, descriptor (Single_Segment, no checksum, no dictionary), content size in 1 / 2 (+256) / 4 bytes
+__host__ __device__ __forceinline__ uint32_t zframe_header_len(uint32_t ulen) { return 5u + (ulen < 256 ? 1u : (ulen < 65536 + 256 ? 2u : 4u)); }
+__host__ __device__ __forceinline__ uint32_t zblocks_of(uint32_t ulen) { return (ulen + kZBlk - 1) / kZBlk; }
+
+__device__ __forceinline__ int hbit(uint32_t v) { return 31 - __clz(int(v)); }      // v > 0
+__device__ __forceinline__ uint32_t zcode_ll(uint32_t v) {
+  if (v < 16) return v;
+  uint32_t lo = 16, hi = zst::kMaxLL - 1;
+  while (lo < hi) { const uint32_t m = (lo + hi + 1) >> 1; if (zst::ll_base(m) <= v) lo = m; else hi = m - 1; }
+  return lo;
+}
+__device__ __forceinline__ uint32_t zcode_ml(uint32_t v) {      // v >= 3
+  if (v < 35) return v - 3;
+  uint32_t lo = 32, hi = zst::kMaxML - 1;
+  while (lo < hi) { const uint32_t m = (lo + hi + 1) >> 1; if (zst::ml_base(m) <= v) lo = m; else hi = m - 1; }
+  return lo;
+}
+
+// FSE encoding table (the inverse of zstd_core.h's fse_build): state table + per-symbol transforms
+struct ZFseCT {
+  uint16_t state[1 << zst::kLLLog];
+  int32_t dnb[64], dfs[64];                     // deltaNbBits, deltaFindState
+  uint32_t log;
+};
+struct ZSmem {
+  uint32_t hash[1 << kZHashLog];
+  ZFseCT ct[3];                                 // literal lengths, offsets, match lengths (the order of the sequence section)
+  uint32_t hist[3][64];
+  int16_t norm[3][64];
+  uint8_t cell_sym[1 << zst::kLLLog];
+  uint32_t w[9];                                // block_scan
+  uint32_t raw;                                 // the block is stored uncompressed
+};
+
+// normalised counts of `total` events: every used symbol >= 1, the sum is 2^L (L >= highbit(symbols used) + 1)
+__device__ void zfse_normalize(const uint32_t* cnt, int nsym, uint32_t total, int L, int16_t* norm) {
+  const uint32_t size = 1u << L;
+  uint32_t sum = 0;
+  int big = 0;
+  for (int s = 0; s < nsym; s++) {
+    uint32_t n = cnt[s] ? uint32_t((uint64_t(cnt[s]) << L) / total) : 0u;
+    if (cnt[s] && n == 0) n = 1;
+    norm[s] = int16_t(n);
+    sum += n;
+    if (cnt[s] > cnt[big]) big = s;
+  }
+  if (sum <= size) { norm[big] = int16_t(norm[big] + int(size - sum)); return; }
+  for (uint32_t excess = sum - size; excess; excess--) {       // the rounded-up rare symbols took too many cells: the largest give back
+    int m = 0;
+    for (int s = 1; s < nsym; s++) if (norm[s] > norm[m]) m = s;
+    norm[m]--;
+  }
+}
+// table description (RFC 8878 4.1.1) of norm[0 .. nsym), nsym - 1 = the last used symbol; returns the bytes written
+__device__ uint32_t zfse_write_ncount(uint8_t* out, const int16_t* norm, int nsym, int L) {
+  uint64_t acc = 0;
+  int nb = 0;
+  uint32_t n = 0;
+  auto put = [&](uint32_t v, int bits) { acc |= uint64_t(v) << nb; nb += bits; while (nb >= 8) { out[n++] = uint8_t(acc); acc >>= 8; nb -= 8; } };
+  put(uint32_t(L - 5), 4);
+  int remaining = 1 << L, s = 0;
+  while (remaining > 0 && s < nsym) {
+    const int p = norm[s++];
+    const uint32_t mx = uint32_t(remaining + 1), v = uint32_t(p + 1);
+    const int bits = hbit(mx) + 1;
+    const uint32_t lower = (1u << (bits - 1)) - 1u, thr = (1u << bits) - 1u - mx;
+    if (v < thr) put(v, bits - 1);
+    else if (v <= lower) put(v, bits);
+    else put(v + thr, bits);
+    remaining -= p;
+    if (p == 0) {
+      int z = 0;
+      while (s + z < nsym && norm[s + z] == 0) z++;
+      s += z;
+      for (; z >= 3; z -= 3) put(3, 2);
+      put(uint32_t(z), 2);
+    }
+  }
+  if (nb) out[n++] = uint8_t(acc);
+  return n;
+}
+// encoding table of norm[0 .. nsym) at accuracy L (norm -1 = "less than one" cell, as in the predefined distributions)
+__device__ void zfse_build_ct(ZFseCT& ct, const int16_t* norm, int nsym, int L, uint8_t* cell_sym) {
+  const uint32_t size = 1u << L, mask = size - 1, step = (size >> 1) + (size >> 3) + 3;
+  uint32_t high = size - 1, cumul[65];
+  cumul[0] = 0;
+  for (int s = 0; s < nsym; s++) {
+    if (norm[s] == -1) { cumul[s + 1] = cumul[s] + 1; cell_sym[high--] = uint8_t(s); }
+    else cumul[s + 1] = cumul[s] + uint32_t(norm[s]);
+  }
+  uint32_t pos = 0;
+  for (int s = 0; s < nsym; s++)
+    for (int i = 0; i < norm[s]; i++) { cell_sym[pos] = uint8_t(s); do { pos = (pos + step) & mask; } while (pos > high); }
+  for (uint32_t u = 0; u < size; u++) ct.state[cumul[cell_sym[u]]++] = uint16_t(size + u);
+  int total = 0;
+  for (int s = 0; s < nsym; s++) {
+    const int c = norm[s];
+    if (c == 0) { ct.dnb[s] = int32_t(((uint32_t(L) + 1) << 16) - size); ct.dfs[s] = 0; }
+    else if (c == -1 || c == 1) { ct.dnb[s] = int32_t((uint32_t(L) << 16) - size); ct.dfs[s] = total - 1; total++; }
+    else {
+      const uint32_t mbo = uint32_t(L - hbit(uint32_t(c - 1)));
+      ct.dnb[s] = int32_t((mbo << 16) - (uint32_t(c) << mbo));
+      ct.dfs[s] = total - c;
+      total += c;
+    }
+  }
+  ct.log = uint32_t(L);
+}
+
+// forward bit writer of the sequence bitstream (read backwards by the decoder); `over` once it would pass `cap`
+struct ZBitW {
+  uint8_t* p; uint32_t n, cap; uint64_t acc; int nb; bool over;
+  __device__ void add(uint32_t v, int bits) {
+    acc |= (uint64_t(v) & ((1ull << bits) - 1ull)) << nb;
+    nb += bits;
+    while (nb >= 8) { if (n < cap) p[n] = uint8_t(acc); else over = true; n++; acc >>= 8; nb -= 8; }
+  }
+};
+__device__ __forceinline__ uint32_t zfse_init(const ZFseCT& ct, uint32_t sym) {
+  const uint32_t nbo = uint32_t(ct.dnb[sym] + (1 << 15)) >> 16;
+  const uint32_t v = (nbo << 16) - uint32_t(ct.dnb[sym]);
+  return ct.state[(v >> nbo) + ct.dfs[sym]];
+}
+__device__ __forceinline__ void zfse_encode(ZBitW& bw, const ZFseCT& ct, uint32_t& st, uint32_t sym) {
+  const uint32_t nbo = (st + uint32_t(ct.dnb[sym])) >> 16;
+  bw.add(st, int(nbo));
+  st = ct.state[(st >> nbo) + ct.dfs[sym]];
+}
+
+// One CTA per (page, 128 KB block).  The block's values (those wholly inside it) are classed like the Snappy path's, plus
+// F(d) = equal to the value d positions back (hash table); runs of equal class become sequences; the level prefix and partial
+// values at the block's edges are literals.  Output: [frame header (block 0)][block header][literals][sequences] in the
+// block's slot of `comp`; zsz[page * nbmax + b] = its bytes (0: no such block).
+__global__ void __launch_bounds__(kThreads) zstd_encode_kernel(const uint8_t* __restrict__ body, uint64_t bstride, const PageMetaDev* __restrict__ meta,
+                                                              const PageJob* __restrict__ jobs, uint32_t ncols, uint32_t nbmax, uint8_t* __restrict__ comp,
+                                                              uint64_t cstride, uint64_t zslot, uint32_t* __restrict__ zsz, uint8_t* __restrict__ scratch,
+                                                              uint64_t sstride, uint32_t vcap) {
+  __shared__ ZSmem sm;
+  const uint32_t page = blockIdx.x / nbmax, b = blockIdx.x % nbmax;
+  const uint32_t w = jobs[page % ncols].pwidth;
+  const uint8_t* in = body + uint64_t(page) * bstride;
+  const uint32_t ulen = meta[page].uncomp_size;
+  const int tid = threadIdx.x;
+  if (b >= zblocks_of(ulen)) { if (tid == 0) zsz[blockIdx.x] = 0; return; }
+  uint8_t* const slot = comp + uint64_t(page) * cstride + uint64_t(b) * zslot;
+  uint8_t* const out = slot + kZFront;                        // block header
+  const uint32_t prefix = 4 + (uint32_t(in[0]) | (uint32_t(in[1]) << 8) | (uint32_t(in[2]) << 16) | (uint32_t(in[3]) << 24));
+  const uint32_t nv = (ulen - prefix) / w;
+  const uint32_t bstart = b * kZBlk, bend = min(bstart + kZBlk, ulen), content = bend - bstart;
+  const bool last = bend == ulen;
+  // values wholly inside the block: [fi, li); head = literal bytes in front of them, tail = behind them
+  const uint32_t fi = bstart <= prefix ? 0u : min(nv, (bstart - prefix + w - 1) / w);
+  uint32_t li = bend <= prefix ? 0u : min(nv, (bend - prefix) / w);
+  if (li < fi) li = fi;
+  const uint32_t nvb = li - fi;
+  const uint32_t head = nvb ? prefix + fi * w - bstart : content, tail = nvb ? bend - (prefix + li * w) : 0u;
+  const uint8_t* v = in + prefix;
+  const bool val_aligned = (prefix & (w - 1)) == 0;
+  auto val_at = [&](uint32_t i) -> uint64_t {
+    if (val_aligned) return w == 8 ? *reinterpret_cast<const uint64_t*>(v + size_t(i) * 8) : uint64_t(*reinterpret_cast<const uint32_t*>(v + size_t(i) * 4));
+    uint64_t x = 0;
+    for (uint32_t k = 0; k < w; k++) x |= uint64_t(v[size_t(i) * w + k]) << (8 * k);
+    return x;
+  };
+  uint32_t* const cd = reinterpret_cast<uint32_t*>(scratch + uint64_t(blockIdx.x) * sstride);   // candidate distance, then run of value
+  uint32_t* const key = cd + vcap;                            // 0 literal, 1..5 P(k): k low bytes + match of 8-k at offset 8, d << 3: F(d)
+  uint32_t* const run_pos = key + vcap;                       // [vcap + 1]
+  uint32_t* const run_lit = run_pos + vcap + 1;               // literal bytes in front of run r (value literals only)
+  uint32_t* const seq_end = run_lit + vcap;                   // literal bytes up to the match of sequence j (head included)
+  uint32_t* const seq_run = seq_end + vcap;
+  uint32_t* const seq_ll = seq_run + vcap;
+  uint32_t* const seq_ml = seq_ll + vcap;
+  uint32_t* const seq_of = seq_ml + vcap;                     // offset + 3
+  uint32_t* const seq_code = seq_of + vcap;                   // LL code | ML code << 8 | OF code << 16
+  for (uint32_t i = tid; i < (1u << kZHashLog); i += kThreads) sm.hash[i] = 0;
+  for (uint32_t i = tid; i < 3 * 64; i += kThreads) sm.hist[i / 64][i % 64] = 0;
+  __syncthreads();
+  // ---- earlier equal values: chunks of 256 look up what the chunks before them inserted (the largest index per slot)
+  for (uint32_t base = 0; base < nvb; base += kThreads) {
+    const uint32_t q = base + tid;
+    uint32_t h = 0;
+    uint64_t x = 0;
+    if (q < nvb) {
+      x = val_at(fi + q);
+      h = uint32_t((x * 0x9E3779B97F4A7C15ull) >> (64 - kZHashLog));
+      const uint32_t c = sm.hash[h];
+      cd[q] = (c && val_at(fi + c - 1) == x) ? q - (c - 1) : 0u;
+    }
+    __syncthreads();
+    if (q < nvb) atomicMax(&sm.hash[h], q + 1);
+    __syncthreads();
+  }
+  // ---- classes
+  for (uint32_t q = tid; q < nvb; q += kThreads) {
+    uint32_t k2 = 0;
+    if (q > 0) {
+      const uint64_t x = val_at(fi + q) ^ val_at(fi + q - 1);
+      if (x == 0) k2 = 1u << 3;
+      else {
+        const uint32_t k = (71u - uint32_t(__clzll((long long)x))) / 8u;
+        const bool p_ok = w == 8 && k <= 5;
+        const uint32_t d = cd[q];
+        // a lone far match is a whole sequence with a long offset: a close partial match is cheaper
+        if (d && !(p_ok && k <= 2 && cd[q - 1] != d && (q + 1 >= nvb || cd[q + 1] != d))) k2 = d << 3;
+        else if (p_ok) k2 = k;
+      }
+    }
+    key[q] = k2;
+  }
+  __syncthreads();
+  // ---- runs: a new run starts where the class changes; P values are runs of their own
+  uint32_t running = 0;
+  for (uint32_t base = 0; base < nvb; base += kThreads) {
+    const uint32_t q = base + tid;
+    uint32_t st = 0;
+    if (q < nvb) { const uint32_t c = key[q]; st = (q == 0 || c != key[q - 1] || (c >= 1 && c < 8)) ? 1u : 0u; }
+    uint32_t total;
+    const uint32_t r = running + block_scan(st, &total, sm.w) + st - 1;
+    if (q < nvb) { cd[q] = r; if (st) run_pos[r] = q; }
+    running += total;
+  }
+  const uint32_t nruns = running;
+  if (tid == 0) run_pos[nruns] = nvb;
+  __syncthreads();
+  // ---- literal bytes and sequences per run
+  uint32_t lrun = 0, srun = 0;
+  for (uint32_t base = 0; base < nruns; base += kThreads) {
+    const uint32_t r = base + tid;
+    uint32_t lit = 0, isseq = 0;
+    if (r < nruns) {
+      const uint32_t a = run_pos[r], c = key[a];
+      lit = c == 0 ? (run_pos[r + 1] - a) * w : (c < 8 ? c : 0u);
+      isseq = c != 0;
+    }
+    uint32_t lt, stot;
+    const uint32_t lo = lrun + block_scan(lit, &lt, sm.w);
+    const uint32_t so = srun + block_scan(isseq, &stot, sm.w);
+    if (r < nruns) {
+      run_lit[r] = lo;
+      if (isseq) { seq_end[so] = head + lo + lit; seq_run[so] = r; }
+    }
+    lrun += lt;
+    srun += stot;
+  }
+  const uint32_t nseq = srun, ltot = head + lrun + tail;
+  __syncthreads();
+  // ---- sequence values and codes
+  for (uint32_t j = tid; j < nseq; j += kThreads) {
+    const uint32_t r = seq_run[j], a = run_pos[r], c = key[a];
+    const uint32_t ll = seq_end[j] - (j ? seq_end[j - 1] : 0u);
+    const uint32_t ml = c < 8 ? 8 - c : (run_pos[r + 1] - a) * w;
+    const uint32_t ofb = (c < 8 ? 8u : (c >> 3) * w) + 3u;
+    const uint32_t llc = zcode_ll(ll), mlc = zcode_ml(ml), ofc = uint32_t(hbit(ofb));
+    seq_ll[j] = ll; seq_ml[j] = ml; seq_of[j] = ofb;
+    seq_code[j] = llc | (mlc << 8) | (ofc << 16);
+    atomicAdd(&sm.hist[0][llc], 1u);
+    atomicAdd(&sm.hist[1][ofc], 1u);
+    atomicAdd(&sm.hist[2][mlc], 1u);
+  }
+  // ---- literals, stored raw: head, the literal bytes of the values, tail
+  const uint32_t lh = ltot < 32 ? 1u : (ltot < 4096 ? 2u : 3u);
+  uint8_t* const lits = out + 3 + lh;
+  for (uint32_t x = tid; x < head; x += kThreads) lits[x] = in[bstart + x];
+  for (uint32_t x = tid; x < tail; x += kThreads) lits[head + lrun + x] = in[prefix + li * w + x];
+  for (uint32_t q = tid; q < nvb; q += kThreads) {
+    const uint32_t c = key[q];
+    if (c >= 8) continue;
+    const uint32_t r = cd[q];
+    const uint8_t* src = v + size_t(fi + q) * w;
+    uint8_t* dst = lits + head + run_lit[r] + (c == 0 ? (q - run_pos[r]) * w : 0u);
+    for (uint32_t k = 0; k < (c == 0 ? w : c); k++) dst[k] = src[k];
+  }
+  __syncthreads();
+  // ---- sequences section: one thread (the FSE states are a serial chain)
+  if (tid == 0) {
+    if (lh == 1) out[3] = uint8_t(ltot << 3);
+    else if (lh == 2) { out[3] = uint8_t(((ltot & 15) << 4) | 4); out[4] = uint8_t(ltot >> 4); }
+    else { out[3] = uint8_t(((ltot & 15) << 4) | 12); out[4] = uint8_t(ltot >> 4); out[5] = uint8_t(ltot >> 12); }
+    uint32_t pos = 3 + lh + ltot;
+    uint8_t* o = out;
+    if (nseq < 128) o[pos++] = uint8_t(nseq);
+    else if (nseq < 0x7f00) { o[pos++] = uint8_t((nseq >> 8) + 128); o[pos++] = uint8_t(nseq); }
+    else { o[pos++] = 255; o[pos++] = uint8_t(nseq - 0x7f00); o[pos++] = uint8_t((nseq - 0x7f00) >> 8); }
+    bool ok = pos < content;
+    uint32_t mode[3] = {0, 0, 0};
+    if (nseq && ok) {
+      const uint32_t mpos = pos++;
+      for (int t = 0; t < 3; t++) {
+        const int nsym = t == 0 ? zst::kMaxLL : (t == 1 ? zst::kMaxOF : zst::kMaxML);
+        const int max_log = t == 0 ? zst::kLLLog : (t == 1 ? zst::kOFLog : zst::kMLLog);
+        const uint32_t* cnt = sm.hist[t];
+        int used = 0, lastsym = 0;
+        for (int s = 0; s < nsym; s++) if (cnt[s]) { used++; lastsym = s; }
+        if (used == 1) { mode[t] = 1; o[pos++] = uint8_t(lastsym); continue; }
+        // predefined distribution: accuracy 6 (5 for offsets), defined up to code 35 / 28 / 52
+        const int dlog = t == 1 ? 5 : 6, dsym = t == 0 ? 36 : (t == 1 ? 29 : 53);
+        uint64_t cost_pre = ~0ull;
+        if (lastsym < dsym) {
+          cost_pre = 0;
+          for (int s = 0; s <= lastsym; s++) {
+            if (!cnt[s]) continue;
+            const int d = t == 0 ? zst::ll_default(s) : (t == 1 ? zst::of_default(s) : zst::ml_default(s));
+            cost_pre += uint64_t(cnt[s]) * uint32_t(dlog - hbit(uint32_t(d < 1 ? 1 : d)));
+          }
+        }
+        int L = hbit(nseq) + 1;
+        L = L < 5 ? 5 : (L > max_log ? max_log : L);
+        if ((1 << L) <= used) L = hbit(uint32_t(used)) + 1;
+        int16_t* norm = sm.norm[t];
+        zfse_normalize(cnt, lastsym + 1, nseq, L, norm);
+        const uint32_t hdr = zfse_write_ncount(o + pos, norm, lastsym + 1, L);
+        uint64_t cost_cmp = uint64_t(hdr) * 8;
+        for (int s = 0; s <= lastsym; s++) if (cnt[s]) cost_cmp += uint64_t(cnt[s]) * uint32_t(L - hbit(uint32_t(norm[s])));
+        if (cost_cmp < cost_pre) { mode[t] = 2; pos += hdr; zfse_build_ct(sm.ct[t], norm, lastsym + 1, L, sm.cell_sym); }
+        else {
+          for (int s = 0; s < dsym; s++) norm[s] = int16_t(t == 0 ? zst::ll_default(s) : (t == 1 ? zst::of_default(s) : zst::ml_default(s)));
+          zfse_build_ct(sm.ct[t], norm, dsym, dlog, sm.cell_sym);
+        }
+      }
+      o[mpos] = uint8_t((mode[0] << 6) | (mode[1] << 4) | (mode[2] << 2));
+      ok = pos < content;
+      if (ok) {
+        ZBitW bw{o + pos, 0, content - pos, 0, 0, false};
+        uint32_t st[3] = {0, 0, 0};
+        const uint32_t c0 = seq_code[nseq - 1];
+        const uint32_t sym_last[3] = {c0 & 0xffu, (c0 >> 16) & 0xffu, (c0 >> 8) & 0xffu};
+        for (int t = 0; t < 3; t++) if (mode[t] != 1) st[t] = zfse_init(sm.ct[t], sym_last[t]);
+        auto extras = [&](uint32_t j, uint32_t code) {
+          const uint32_t llc = code & 0xffu, mlc = (code >> 8) & 0xffu, ofc = (code >> 16) & 0xffu;
+          bw.add(seq_ll[j] - zst::ll_base(llc), int(zst::ll_bits(llc)));
+          bw.add(seq_ml[j] - zst::ml_base(mlc), int(zst::ml_bits(mlc)));
+          bw.add(seq_of[j], int(ofc));
+        };
+        extras(nseq - 1, c0);
+        for (uint32_t j = nseq - 1; j-- > 0 && !bw.over;) {
+          const uint32_t c = seq_code[j];
+          if (mode[1] != 1) zfse_encode(bw, sm.ct[1], st[1], (c >> 16) & 0xffu);
+          if (mode[2] != 1) zfse_encode(bw, sm.ct[2], st[2], (c >> 8) & 0xffu);
+          if (mode[0] != 1) zfse_encode(bw, sm.ct[0], st[0], c & 0xffu);
+          extras(j, c);
+        }
+        if (mode[2] != 1) bw.add(st[2], int(sm.ct[2].log));
+        if (mode[1] != 1) bw.add(st[1], int(sm.ct[1].log));
+        if (mode[0] != 1) bw.add(st[0], int(sm.ct[0].log));
+        bw.add(1, 1);                                         // end mark
+        if (bw.nb) { if (bw.n < bw.cap) bw.p[bw.n] = uint8_t(bw.acc); else bw.over = true; bw.n++; }
+        pos += bw.n;
+        ok = !bw.over && pos - 3 < content;
+      }
+    }
+    ok = ok && pos - 3 < content;
+    const uint32_t bsize = ok ? pos - 3 : content;
+    const uint32_t bh = (last ? 1u : 0u) | ((ok ? 2u : 0u) << 1) | (bsize << 3);
+    out[0] = uint8_t(bh); out[1] = uint8_t(bh >> 8); out[2] = uint8_t(bh >> 16);
+    sm.raw = ok ? 0u : 1u;
+    uint32_t n = 3 + bsize;
+    if (b == 0) {
+      const uint32_t fh = zframe_header_len(ulen);
+      uint8_t* f = out - fh;
+      f[0] = 0x28; f[1] = 0xb5; f[2] = 0x2f; f[3] = 0xfd;
+      if (ulen < 256) { f[4] = 0x20; f[5] = uint8_t(ulen); }
+      else if (ulen < 65536 + 256) { f[4] = 0x60; f[5] = uint8_t(ulen - 256); f[6] = uint8_t((ulen - 256) >> 8); }
+      else { f[4] = 0xa0; for (int k = 0; k < 4; k++) f[5 + k] = uint8_t(ulen >> (8 * k)); }
+      n += fh;
+    }
+    zsz[blockIdx.x] = n;
+  }
+  __syncthreads();
+  if (sm.raw) for (uint32_t x = tid; x < content; x += kThreads) out[3 + x] = in[bstart + x];
+}
+
 struct GatherDesc { uint64_t src_off, dst_off; uint32_t bytes, _pad; };
 __global__ void __launch_bounds__(kThreads) gather_pages_kernel(const uint8_t* __restrict__ src, const GatherDesc* __restrict__ d, uint8_t* __restrict__ file) {
   const GatherDesc g = d[blockIdx.x];
@@ -387,8 +791,9 @@ int write_sst(hg_engine* e, const hg_schema_desc* schema, const ColIn* cols, uin
               uint8_t** host_out, uint64_t* size_out) {
   cudaStream_t s = e->stream;
   const uint32_t rg_rows = props->max_row_group_size ? props->max_row_group_size : 8192;
-  const bool snappy = props->compression == 1;
-  if (props->compression > 1) return set_error(HG_ERR_UNSUPPORTED, "write: only UNCOMPRESSED and SNAPPY pages are implemented");
+  const uint32_t codec = props->compression;
+  const bool snappy = codec == 1, zstd = codec == 6;
+  if (codec != 0 && !snappy && !zstd) return set_error(HG_ERR_UNSUPPORTED, "write: only UNCOMPRESSED, SNAPPY and ZSTD pages are implemented");
   const uint32_t nrg = (R + rg_rows - 1) / rg_rows;
   const uint64_t npages = uint64_t(nrg) * ncols;
   std::vector<PageJob> jobs(ncols);
@@ -399,8 +804,15 @@ int write_sst(hg_engine* e, const hg_schema_desc* schema, const ColIn* cols, uin
   const uint64_t bstride = (uint64_t(16) + (max_vals + 7) / 8 + 8 + uint64_t(max_vals) * 8 + 63) & ~uint64_t(63);
   const uint64_t cstride = bstride + 64;
   const uint64_t sstride = ((uint64_t(max_vals) + 15) & ~uint64_t(15)) + (uint64_t(max_vals) * 3 + 4) * 4;
-  DevBuf d_jobs, d_body, d_comp, d_meta, d_scratch;
+  // Zstandard: one slot per 128 KB block of a page (a page never exceeds bstride bytes); scratch per (page, block)
+  const uint32_t nbmax = zblocks_of(uint32_t(std::min<uint64_t>(bstride, 0xffffffffull)));
+  const uint32_t vcap = std::min<uint32_t>(max_vals, kZBlk / 4);
+  const uint64_t zslot = (kZFront + 3 + std::min<uint64_t>(bstride, kZBlk) + kZPad + 63) & ~uint64_t(63);
+  const uint64_t zcstride = nbmax * zslot;
+  const uint64_t zsstride = (uint64_t(kZArrays) * vcap * 4 + 4 + 63) & ~uint64_t(63);
+  DevBuf d_jobs, d_body, d_comp, d_meta, d_scratch, d_zsz;
   std::vector<PageMetaDev> meta(npages);
+  std::vector<uint32_t> zsz(zstd ? npages * nbmax : 0);
   if (npages) {
     CU_TRY(d_jobs.alloc(jobs.size() * sizeof(PageJob), s));
     CU_TRY(d_body.alloc(npages * bstride, s));
@@ -415,14 +827,29 @@ int write_sst(hg_engine* e, const hg_schema_desc* schema, const ColIn* cols, uin
       snappy_encode_kernel<<<uint32_t(npages), kThreads, 0, s>>>(d_body.as<uint8_t>(), bstride, d_meta.as<PageMetaDev>(), d_jobs.as<PageJob>(), ncols,
                                                                 d_comp.as<uint8_t>(), cstride, d_scratch.as<uint8_t>(), sstride, max_vals);
       e->launches++;
+    } else if (zstd) {
+      CU_TRY(d_comp.alloc(npages * zcstride, s));
+      CU_TRY(d_scratch.alloc(npages * nbmax * zsstride, s));
+      CU_TRY(d_zsz.alloc(npages * nbmax * sizeof(uint32_t), s));
+      zstd_encode_kernel<<<uint32_t(npages * nbmax), kThreads, 0, s>>>(d_body.as<uint8_t>(), bstride, d_meta.as<PageMetaDev>(), d_jobs.as<PageJob>(), ncols, nbmax,
+                                                                      d_comp.as<uint8_t>(), zcstride, zslot, d_zsz.as<uint32_t>(), d_scratch.as<uint8_t>(), zsstride, vcap);
+      e->launches++;
+      CU_TRY(cudaMemcpyAsync(zsz.data(), d_zsz.p, zsz.size() * sizeof(uint32_t), cudaMemcpyDeviceToHost, s));
     }
     CU_TRY(cudaGetLastError());
     CU_TRY(cudaMemcpyAsync(meta.data(), d_meta.p, npages * sizeof(PageMetaDev), cudaMemcpyDeviceToHost, s));
     CU_TRY(cudaStreamSynchronize(s));
+    if (zstd)
+      for (uint64_t p = 0; p < npages; p++) {
+        uint64_t c = 0;
+        for (uint32_t b = 0; b < nbmax; b++) c += zsz[p * nbmax + b];
+        meta[p].comp_size = uint32_t(c);
+      }
   }
   // ---- host: page headers, offsets, footer
   std::vector<std::vector<uint8_t>> headers(npages);
-  std::vector<GatherDesc> gd(npages);
+  std::vector<GatherDesc> gd;
+  gd.reserve(npages);
   std::vector<uint64_t> hdr_off(npages);
   uint64_t pos = 4;
   for (uint64_t p = 0; p < npages; p++) {
@@ -443,7 +870,17 @@ int write_sst(hg_engine* e, const hg_schema_desc* schema, const ColIn* cols, uin
     headers[p] = std::move(t.b);
     hdr_off[p] = pos;
     pos += headers[p].size();
-    gd[p] = GatherDesc{p * (snappy ? cstride : bstride), pos, meta[p].comp_size, 0};
+    if (zstd) {                            // the frame: its blocks' slots, the frame header in front of block 0
+      uint64_t at = pos;
+      for (uint32_t b = 0; b < nbmax; b++) {
+        const uint32_t n = zsz[p * nbmax + b];
+        if (!n) continue;
+        gd.push_back(GatherDesc{p * zcstride + b * zslot + kZFront - (b == 0 ? zframe_header_len(meta[p].uncomp_size) : 0u), at, n, 0});
+        at += n;
+      }
+    } else {
+      gd.push_back(GatherDesc{p * (snappy ? cstride : bstride), pos, meta[p].comp_size, 0});
+    }
     pos += meta[p].comp_size;
   }
   TOut f;
@@ -482,7 +919,7 @@ int write_sst(hg_engine* e, const hg_schema_desc* schema, const ColIn* cols, uin
       f.i32(1, phys_of(cols[c].type));
       f.list(2, 5, 2); f.svar(0); f.svar(3);      // encodings: PLAIN, RLE
       f.list(3, 8, 1); f.list_str(schema->names && schema->names[c] ? std::string(schema->names[c]) : "c" + std::to_string(c));
-      f.i32(4, snappy ? 1 : 0);
+      f.i32(4, int(codec));
       f.i64(5, rows);
       f.i64(6, int64_t(meta[p].uncomp_size + hsz));
       f.i64(7, int64_t(meta[p].comp_size + hsz));
@@ -511,7 +948,7 @@ int write_sst(hg_engine* e, const hg_schema_desc* schema, const ColIn* cols, uin
     f.field(7, 4); f.svar(g);              // ordinal (i16)
     f.end();
   }
-  f.str(6, "horaedb_b200 GPU SST writer (PLAIN, RLE levels, " + std::string(snappy ? "SNAPPY" : "UNCOMPRESSED") + ")");
+  f.str(6, "horaedb_b200 GPU SST writer (PLAIN, RLE levels, " + std::string(snappy ? "SNAPPY" : (zstd ? "ZSTD" : "UNCOMPRESSED")) + ")");
   f.list(7, 12, ncols);                    // column_orders: TYPE_ORDER for every column (makes min_value / max_value usable)
   for (uint32_t c = 0; c < ncols; c++) { f.begin(); f.struct_field(1); f.end(); f.end(); }
   f.end();
@@ -527,7 +964,7 @@ int write_sst(hg_engine* e, const hg_schema_desc* schema, const ColIn* cols, uin
   if (npages) {
     CU_TRY(d_gd.alloc(gd.size() * sizeof(GatherDesc), s));
     CU_TRY(cudaMemcpyAsync(d_gd.p, gd.data(), gd.size() * sizeof(GatherDesc), cudaMemcpyHostToDevice, s));
-    gather_pages_kernel<<<uint32_t(npages), kThreads, 0, s>>>(snappy ? d_comp.as<uint8_t>() : d_body.as<uint8_t>(), d_gd.as<GatherDesc>(), d_file.as<uint8_t>());
+    gather_pages_kernel<<<uint32_t(gd.size()), kThreads, 0, s>>>(snappy || zstd ? d_comp.as<uint8_t>() : d_body.as<uint8_t>(), d_gd.as<GatherDesc>(), d_file.as<uint8_t>());
     e->launches++;
     CU_TRY(cudaMemcpyAsync(host + 4, d_file.as<uint8_t>() + 4, footer_off - 4, cudaMemcpyDeviceToHost, s));
     CU_TRY(cudaStreamSynchronize(s));

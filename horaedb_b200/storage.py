@@ -132,7 +132,7 @@ class ObjectBasedStorage:
         w = self.config.write
         gpu_writer = (hasattr(self.engine, "write_batch") and w.encoding == "PLAIN" and not w.enable_dict and not w.column_options
                       and not any(pa.types.is_binary(f.type) for f in self.schema_.arrow_schema)
-                      and str(w.compression).lower() in ("snappy", "uncompressed", "none")
+                      and str(w.compression).lower() in ("snappy", "zstd", "uncompressed", "none")
                       and all(req.batch.column(i).null_count == 0 for i in range(self.schema_.num_primary_keys)))
         if gpu_writer:
             # write_batch on the GPU (hg_write_batch): PK sort, builtin columns, Parquet encode
@@ -140,7 +140,7 @@ class ObjectBasedStorage:
                                            compression=str(w.compression), enable_sorting_columns=w.enable_sorting_columns)
             size = meta.size
         else:
-            # writer options the GPU encoder does not implement (dictionary / delta encodings, zstd, NULL keys): host Parquet writer
+            # writer options the GPU encoder does not implement (dictionary / delta encodings, NULL keys): host Parquet writer
             data = sstgen.write_sst(self.schema_, req.batch, file_id, self.config.write)
             with open(fpath, "wb") as f:
                 f.write(data)
@@ -196,7 +196,7 @@ class ObjectBasedStorage:
                 time_range.merge(f.meta().time_range)
             file_id = allocate_id()
             w = self.config.write
-            if (w.encoding == "PLAIN" and not w.enable_dict and not w.column_options and str(w.compression).lower() in ("snappy", "uncompressed", "none")
+            if (w.encoding == "PLAIN" and not w.enable_dict and not w.column_options and str(w.compression).lower() in ("snappy", "zstd", "uncompressed", "none")
                     and not any(pa.types.is_binary(f.type) for f in self.schema_.arrow_schema)):
                 # the whole of do_compaction on the GPU: merge + dedup (keep_builtin = true) AND the Parquet encode (hg_compact_to_sst)
                 meta = self.engine.compact_to_sst(self.handle, self._inputs(task.inputs), self.sst_path_gen.generate(file_id),
@@ -204,7 +204,7 @@ class ObjectBasedStorage:
                                                   enable_sorting_columns=w.enable_sorting_columns)
                 num_rows, size = meta.num_rows, meta.size
             else:
-                # writer options the GPU encoder does not implement (dictionary / delta encodings, zstd ..): the merged stream comes
+                # writer options the GPU encoder does not implement (dictionary / delta encodings ..): the merged stream comes
                 # back as Arrow batches (hg_compact_open) and the host writes the file, like the reference's AsyncArrowWriter
                 reader = self.engine.compact(self.handle, self._inputs(task.inputs))   # same plan, keep_builtin=true
                 tbl = reader.read_all()

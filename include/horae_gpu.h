@@ -176,8 +176,8 @@ int hg_compact_open(hg_engine* e, const hg_schema_desc* schema, const hg_sst_des
  * PLAIN values, RLE definition levels, dictionary off, bloom filters off, chunk statistics on, one DataPage V1 per chunk. */
 typedef struct {
   uint32_t max_row_group_size;      /* 0 = 8192 (WriteConfig::default) */
-  uint32_t compression;             /* Parquet codec id the WRITER applies: 0 UNCOMPRESSED, 1 SNAPPY (the default).  Readers also take 6 = ZSTD
-                                       (config.rs:78-94: Uncompressed / Snappy / Zstd); Zstd SSTs run on the general pipeline */
+  uint32_t compression;             /* Parquet codec id the WRITER applies (config.rs:78-94): 0 UNCOMPRESSED, 1 SNAPPY (the default),
+                                       6 ZSTD (one frame per page, blocks of <= 128 KB).  Zstd SSTs are read on the general pipeline */
   uint32_t enable_sorting_columns;  /* sorting_columns = primary keys, ascending, nulls first */
   uint32_t _pad;
 } hg_write_props;
